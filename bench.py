@@ -5,6 +5,7 @@ lineitem, the metric BASELINE.json names: rows/s + achieved HBM GB/s, next to th
   python bench.py [--gpus N] [--steps K] [--warmup W] [--sf 100]           (our arm)
   python bench.py --impl reference [...]                                     (CPU arm: Arrow/Acero)
   torchrun --nproc-per-node N bench.py --gpus N ...                          (one rank per GPU, NCCL)
+  python bench.py [...] --dump-outputs DIR     (also writes the last timed step's Q1 result as DIR/*.npy)
 
 A step = one pass of Q1 over this rank's lineitem shard.  Weak scaling: every rank holds its own
 SF-`sf` shard (600 037 902 rows at SF-100, 22.8 GB of Q1 columns resident in HBM); the only data-path
@@ -147,6 +148,15 @@ def run_reference(args):
     print(json.dumps(line), flush=True)
 
 
+def dump_outputs(out_dir: str, arrays: dict):
+    """Writes each tensor as out_dir/<name>.npy in float64 (the Q1 counts stay exact: they are far below 2^53), so that
+    two builds can be compared output for output on the same seeded inputs."""
+    import numpy as np
+    os.makedirs(out_dir, exist_ok=True)
+    for name, t in arrays.items():
+        np.save(os.path.join(out_dir, f"{name}.npy"), t.detach().cpu().numpy().astype(np.float64))
+
+
 def bind_to_gpu_numa_node(local: int):
     """Pin this rank's host threads to the CPUs of its GPU's NUMA node BEFORE any pinned buffer is allocated (first touch puts
     the pages there): at 8 ranks the end-to-end leg moves 8 x 55 GB/s out of host memory, and buffers on the wrong socket cross
@@ -271,6 +281,8 @@ def run_ours(args):
             dist.all_reduce(state.acc); dist.all_reduce(state.cnt)
     t_end.record()
     barrier()
+    if args.dump_outputs and rank == 0:                # the last timed step's result, before any untimed step touches it
+        dump_outputs(args.dump_outputs, {"q1_sums": state.acc, "q1_counts": state.cnt})
     total_ms = t_start.elapsed_time(t_end)
     kern_ms = sum(a.elapsed_time(b) for a, b in kev) / args.steps
     launches = ops.launch_count() - launches0
@@ -786,6 +798,9 @@ def main():
     ap.add_argument("--q3-sf", type=float, default=100)
     ap.add_argument("--q3-steps", type=int, default=3)
     ap.add_argument("--no-cpu", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write the Q1 state of the last timed step as DIR/q1_sums.npy (6 groups x 5 sums, "
+                         "group = returnflag * 2 + linestatus) and DIR/q1_counts.npy, both float64 (rank 0)")
     ap.add_argument("--chunk-rows", type=int, default=0,
                     help="Q3 / Q5 readers emit chunks of this many rows (0 = one batch per shard); chunks are pipelined over lanes")
     args = ap.parse_args()

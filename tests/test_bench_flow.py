@@ -88,9 +88,10 @@ def test_parquet_leg(bench_on_shim):
         assert r[f"file_bytes_{codec}"] > 0
 
 
-def test_headline_line(bench_on_shim, monkeypatch, capsys):
+def test_headline_line(bench_on_shim, monkeypatch, capsys, tmp_path):
     """The default (headline) arm: warm-up, timed loop with events, untimed extra steps for the clock sampler, parity
-    check, JSON line with every contract key.  CUDA events / devices are faked; the e2e leg (pinned memory) is off."""
+    check, JSON line with every contract key, the last timed step's Q1 state written by --dump-outputs.  CUDA events /
+    devices are faked; the e2e leg (pinned memory) is off."""
     import json
     import quokka_b200
 
@@ -107,7 +108,8 @@ def test_headline_line(bench_on_shim, monkeypatch, capsys):
     monkeypatch.setenv("WORLD_SIZE", "1")
     args = types.SimpleNamespace(sf=0.01, steps=3, warmup=3, variant=0, no_e2e=True, no_q3=False, no_cpu=False, extras=1, cpu_rows=200_000,
                                  only_q3=False, only_asof=False, only_q5=False, only_parquet=False, q3_sf=0.01, q3_steps=1, replicate_builds=False, no_replicate_builds=False,
-                                 asof_quotes=10_000, e2e_rows=1000, e2e_chunk=1000, parquet_sf=0.01, chunk_rows=0, q5_sf=0.01, no_parquet=False)
+                                 asof_quotes=10_000, e2e_rows=1000, e2e_chunk=1000, parquet_sf=0.01, chunk_rows=0, q5_sf=0.01, no_parquet=False,
+                                 dump_outputs=str(tmp_path / "out"))
     bench_on_shim.run_ours(args)
     line = json.loads(capsys.readouterr().out.strip().splitlines()[-1])
     for key in ("metric", "value", "unit", "n_gpus", "steps", "warmup", "ms_per_step", "higher_is_better", "scaling", "vs_baseline", "dtype",
@@ -116,3 +118,8 @@ def test_headline_line(bench_on_shim, monkeypatch, capsys):
     assert line["metric"] == "tpch_q1_rows_per_s" and line["n_gpus"] == 1 and line["steps"] == 3 and line["scaling"] == "weak"
     assert line["parity"]["ok"] is True and line["roofline"]["bound"] == "hbm" and line["cpu_baseline"]["kind"] == "port"
     assert "error" not in (line["q3"] or {}) and "error" not in (line["q5"] or {}) and "error" not in (line["asof"] or {})
+    sums, counts = (np.load(str(tmp_path / "out" / f"{n}.npy")) for n in ("q1_sums", "q1_counts"))
+    assert sums.dtype == counts.dtype == np.float64 and sums.shape == (6, 5) and counts.shape == (6,)
+    assert int(counts.sum()) == line["parity"]["sum_of_group_counts"] == line["parity"]["rows_passing_filter"]
+    li = G.gen_lineitem(0.01, columns=["l_shipdate", "l_quantity"])
+    assert np.isclose(sums[:, 0].sum(), li["l_quantity"][li["l_shipdate"] <= G.DAY_1998_09_02].sum(), rtol=1e-12)

@@ -287,13 +287,12 @@ def test_corrupt_chunks_fail_cleanly(tmp_path):
     assert outcomes["error"] > 40 and outcomes["ok"] + outcomes["error"] == 480, outcomes
 
 
-def test_files_from_an_old_writer():
-    """Files another writer produced (parquet-cpp 1.3, 2017: Snappy, PLAIN_DICTIONARY ids), shipped with pyarrow's tests."""
+def test_files_from_an_old_writer(golden_dir):
+    """Files another writer produced (parquet-cpp 1.3, 2017: Snappy, PLAIN_DICTIONARY ids), from pyarrow's test data."""
     import glob
     import os
-    files = sorted(glob.glob(os.path.join(os.path.dirname(pa.__file__), "tests", "data", "parquet", "v0.7.1*.parquet")))
-    if not files:
-        pytest.skip("pyarrow's test data is not installed")
+    files = sorted(glob.glob(os.path.join(golden_dir, "parquet_v0.7.1", "v0.7.1*.parquet")))
+    assert len(files) == 4
     for f in files:
         names = pq.ParquetFile(f).schema_arrow.names
         P.same(P.read(f, CPU, names), pq.read_table(f, columns=names).replace_schema_metadata(None))
